@@ -13,6 +13,8 @@ With --gpus N > 1 (torchrun, one rank per GPU) every rank runs the same shape on
 strong splits ONE C3 + C2 batch over the ranks by bytes instead), the static Huffman tables are broadcast once over NCCL,
 and rank 0 reports total units / max-over-ranks time.
 --impl reference times the CPU restatement of the reference (oracle/, all host threads) on the SAME buffers and mix.
+--steps K times K steps (resident, end to end and per kernel); --dump-outputs DIR writes what the last resident step computed
+to DIR as .npy files (the inputs are generated from fixed seeds, so two builds can be compared output for output).
 --config c4 / c5 run BASELINE.json's configs 4 (one 2 GiB log stream through GZipOutputStream's bytes) and 5 (level x size
 grid); they print their own JSON line and are not the driver's bench line.
 """
@@ -266,7 +268,11 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--small", action="store_true", help="1/8 size workload for quick checks (not a bench value)")
     ap.add_argument("--no-probe", dest="no_probe", action="store_true", help="(accepted for older command lines; no effect)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -283,6 +289,29 @@ def main():
         run_multi(args, rank, out)
         return
     run_bench(args, rank, local_rank, world, out)
+
+
+DUMP_SEED, DUMP_DEFLATE_STREAMS, DUMP_INFLATE_STREAMS = 20240601, 32, 4
+
+
+def dump_outputs(dirname, dplan, iplan, d_dout, d_dlen, d_dst, d_iout, d_ilen, d_ist, d_iused):
+    """What the two plans handed their caller in the last step, as DIR/<name>.npy: every stream's output length, status and
+    (inflate) input bytes consumed in float64, and the output bytes of a fixed, seeded sample of streams (32 compressed, 4
+    inflated; back to back in stream order) in float32 -- at most 55 MB, so that two builds can be compared output for output."""
+    rng = np.random.default_rng(DUMP_SEED)
+    dlen, ilen = d_dlen.cpu().numpy(), d_ilen.cpu().numpy()
+    dpick = np.sort(rng.choice(dlen.size, min(DUMP_DEFLATE_STREAMS, dlen.size), replace=False))
+    ipick = np.sort(rng.choice(ilen.size, min(DUMP_INFLATE_STREAMS, ilen.size), replace=False))
+
+    def streams(d_buf, offsets, lens, pick):
+        return np.concatenate([d_buf[int(offsets[i]):int(offsets[i] + lens[i])].cpu().numpy() for i in pick]).astype(np.float32)
+    arrays = {"deflate_out_len": dlen, "deflate_status": d_dst.cpu().numpy(), "deflate_sample_streams": dpick,
+              "deflate_out_sample": streams(d_dout, dplan.out_offsets, dlen, dpick),
+              "inflate_out_len": ilen, "inflate_status": d_ist.cpu().numpy(), "inflate_in_used": d_iused.cpu().numpy(),
+              "inflate_sample_streams": ipick, "inflate_out_sample": streams(d_iout, iplan.out_offsets, ilen, ipick)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 def run_bench(args, rank, local_rank, world, out):
@@ -395,6 +424,8 @@ def run_bench(args, rank, local_rank, world, out):
         sampler.start()
     ms_total = timed(step_resident, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the per-kernel timing below runs the plans again
+        dump_outputs(args.dump_outputs, dplan, iplan, d_dout, d_dlen, d_dst, d_iout, d_ilen, d_ist, d_iused)
     ms_step = ms_total / args.steps
     units_t = torch.tensor([float(U_def + U_inf)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -406,7 +437,7 @@ def run_bench(args, rank, local_rank, world, out):
     dplan.set_timing(True)
     iplan.set_timing(True)
     acc = {}
-    reps = max(3, min(args.steps, 5))
+    reps = args.steps
     for _ in range(reps):
         step_resident(overlap=False)  # one kernel at a time: these are per-kernel durations
         torch.cuda.synchronize()
@@ -492,7 +523,7 @@ def run_bench(args, rank, local_rank, world, out):
     hi = h_iout.numpy()
     for i in range(0, n_inf, max(1, n_inf // 8)):
         assert np.array_equal(hi[iout_off[i]:iout_off[i] + t_np[i].size], t_np[i]), "e2e inflate mismatch %d" % i
-    n_e2e = max(3, args.steps)
+    n_e2e = args.steps
     ms_e2e = timed_host(e2e_steps, n_e2e) / n_e2e
     e2e_val = units / (ms_e2e / 1e3) / 1e9
     # the same call on PAGEABLE host memory (what a caller that never pinned anything hands over): staged by the library
@@ -504,7 +535,7 @@ def run_bench(args, rank, local_rank, world, out):
     dout_p = P.pointers([pg_dout.ctypes.data + int(o) for o in dout_off])
     iout_p = P.pointers([pg_iout.ctypes.data + int(o) for o in iout_off])
     e2e_steps(2)
-    ms_pg = timed_host(e2e_steps, 3) / 3
+    ms_pg = timed_host(e2e_steps, args.steps) / args.steps
     dpipe.close()
     ipipe.close()
     del h_din, h_iin, h_dout, h_iout, pg_dout, pg_iout

@@ -2,7 +2,8 @@
 # Builds libb200z.so in-tree for sm_100a (nvcc cross-compiles without a GPU).
 set -e
 cd "$(dirname "$0")"
-NVCC=${NVCC:-nvcc}
+# nvcc from $NVCC, else PATH, else the toolkit under $CUDA_HOME (default /usr/local/cuda), which a plain login PATH lacks
+NVCC=${NVCC:-$(command -v nvcc || echo "${CUDA_HOME:-/usr/local/cuda}/bin/nvcc")}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -Wall -diag-suppress 550"
 mkdir -p _build
 pids=()
