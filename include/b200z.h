@@ -156,6 +156,11 @@ int b200z_plan_get_restart_points(b200z_plan *plan, int64_t *bit, int64_t *out_p
  * decoded, v[4] rounds, v[5] speculative passes over them, v[6] streams handed back to the serial kernel, v[7] 1 if the
  * plan runs the block-parallel pipeline.  Mirrors nothing in the reference. */
 int b200z_plan_get_stats(b200z_plan *plan, uint32_t *v, int32_t cap, void *cuda_stream);
+/* What the last SEARCH stage of a level 5-9 deflate plan left for stream i (synchronises `stream`), for tests that check
+ * the match search entry for entry: link[hist_len[i] + in_len[i]] (uint16, may be NULL) the hash-chain links of every
+ * position of the slot, history first (0 = no predecessor), and ab[2 * in_len[i]] (uint32) the (A, B) table entries of the
+ * data positions (A: best match with the full chain budget, B: with a quarter of it; len << 16 | dist, 0 = none). */
+int b200z_plan_get_match_table(b200z_plan *plan, int32_t i, uint16_t *link, uint32_t *ab, void *cuda_stream);
 int b200z_plan_destroy(b200z_plan *plan);
 int64_t b200z_plan_in_bytes(const b200z_plan *plan);          /* size of the input blob  */
 int64_t b200z_plan_out_bytes(const b200z_plan *plan);         /* size of the output blob */

@@ -78,6 +78,7 @@ _SIGS = {
     "b200z_plan_get_restart_points": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200z_inflate_plan_set_lengths": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200z_plan_get_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "b200z_plan_get_match_table": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200z_plan_data_offset": (C.c_int64, [C.c_void_p, C.c_int32]),
     "b200z_plan_destroy": (C.c_int, [C.c_void_p]),
     "b200z_plan_in_bytes": (C.c_int64, [C.c_void_p]),

@@ -554,6 +554,15 @@ int b200z_plan_get_stats(b200z_plan *plan, uint32_t *v, int32_t cap, void *cuda_
 	return inflate_plan_stats(plan, v, cap, (cudaStream_t)cuda_stream);
 }
 
+int b200z_plan_get_match_table(b200z_plan *plan, int32_t i, uint16_t *link, uint32_t *ab, void *cuda_stream) {
+	DeviceGuard guard(plan ? plan->device : -1);
+	if (!plan || plan->kind != 0 || plan->level < 5 || i < 0 || i >= plan->n || !ab) {
+		set_error("bad arguments");
+		return B200Z_E_ARG;
+	}
+	return deflate_plan_match_table(plan, i, link, ab, (cudaStream_t)cuda_stream);
+}
+
 int b200z_plan_set_timing(b200z_plan *plan, int enable) {
 	if (!plan) return B200Z_E_ARG;
 	plan->timing = enable != 0;

@@ -19,6 +19,7 @@ constexpr int kTile = 32768;   // positions per k_match CTA
 constexpr int kTileData = 2 * kTile + 320; // bytes of window staged per tile (history + tile + max match + pad)
 constexpr int kMatchThreads = 1024;
 constexpr int kMatchClasses = 16; // expected-walk-length classes of k_match (0 = nothing to search)
+constexpr uint32_t kNoLink = 0xFFFFu; // k_match's staged link entry for "no predecessor": exceeds kMaxDist from any distance
 
 // ------------------------------------------------------------------------------------------------
 // K1: link[p] = distance from p to the previous inserted position with the same hash (0 = none / too far).
@@ -190,6 +191,15 @@ __global__ void __launch_bounds__(kMatchThreads, 1)
 	}
 	bulk_wait(&s_bar, 0);
 	__syncthreads();
+	// k_links writes 0 for "no predecessor"; here it becomes kNoLink, so that the end of a chain and the T7 limit are one test,
+	// dist + l2 >= kMaxDist.  (The entry past an odd nl is never read.)
+	for (uint32_t i = threadIdx.x; i < (t1 - w0 + 1) / 2; i += kMatchThreads) {
+		const uint32_t v = reinterpret_cast<uint32_t *>(s_link)[i];
+		reinterpret_cast<uint32_t *>(s_link)[i] = v | ((v & 0xFFFFu) ? 0u : kNoLink) | ((v >> 16) ? 0u : kNoLink << 16);
+	}
+	__shared__ uint32_t s_cls[2][kMatchClasses];
+	if (threadIdx.x < 2 * kMatchClasses) (&s_cls[0][0])[threadIdx.x] = 0;
+	__syncthreads(); // the class pass reads entries other threads rewrote
 	uint2 *out = mt + off;
 	// match_search() of b200z_core.cuh with the byte-wise extension loop replaced by 4-byte compares on aligned
 	// shared-memory words (ncu: the byte loop ran with ~2 of 32 lanes active and took ~30 % of the kernel).
@@ -204,9 +214,6 @@ __global__ void __launch_bounds__(kMatchThreads, 1)
 	// (Measured in round 2 and dropped: the walks as a flat state machine -- one candidate test or four bytes of extension per
 	// lane and iteration, free lanes refilled from the ordered list eight at a time.  Bit-exact, 41.5 ms instead of 21.2 ms on
 	// the bench workload: every iteration pays for every state's code.  profiles/README.md.)
-	__shared__ uint32_t s_cls[2][kMatchClasses];
-	if (threadIdx.x < 2 * kMatchClasses) (&s_cls[0][0])[threadIdx.x] = 0;
-	__syncthreads();
 	uint16_t *order = reinterpret_cast<uint16_t *>(scratch + off + t0); // 4 bytes per position are free here until k_parse_gather
 	uint32_t cw[4] = {0u, 0u, 0u, 0u};                                   // 32 x 4 bits: this thread's classes
 	const int lane = threadIdx.x & 31;
@@ -216,15 +223,14 @@ __global__ void __launch_bounds__(kMatchThreads, 1)
 		uint32_t cls = 0;
 		if (p < t1 && p >= H) {
 			const uint32_t la = n - p;
-			uint32_t d = la >= (uint32_t)kMinMatch ? (uint32_t)s_link[p - w0] : 0u;
-			if (d > (uint32_t)kMaxDist - (is_slide_pos(p + ab) ? 1u : 0u)) d = 0; // DeflaterEngine.cs:788 + trap T8
-			if (d == 0) out[p] = make_uint2(0u, 0u);
+			const uint32_t d = la >= (uint32_t)kMinMatch ? (uint32_t)s_link[p - w0] : kNoLink;
+			if (d > (uint32_t)kMaxDist - (is_slide_pos(p + ab) ? 1u : 0u)) out[p] = make_uint2(0u, 0u); // DeflaterEngine.cs:788 + trap T8
 			else {
 				const uint32_t is = p - w0;
 				uint32_t dist = d, hops = 1;
 				while (hops < 8) {
 					const uint32_t l2 = s_link[is - dist];
-					if (l2 == 0 || dist + l2 >= (uint32_t)kMaxDist) break;
+					if (dist + l2 >= (uint32_t)kMaxDist) break;
 					dist += l2;
 					++hops;
 				}
@@ -267,88 +273,96 @@ __global__ void __launch_bounds__(kMatchThreads, 1)
 		if (cls) order[slot + (uint32_t)__popc(peers & ((1u << lane) - 1u))] = (uint16_t)(threadIdx.x + (uint32_t)k * kMatchThreads);
 	}
 	__syncthreads();
+	// The walk keeps two running byte offsets into shared memory, both moved by each hop: icm, of the candidate's byte c[m], and il,
+	// of the candidate's link entry (il = 2 * ic); the next hop's link is loaded before the quick reject, so the two shared-memory
+	// latencies overlap.  The end of the chain (kNoLink) and the T7 limit are the one test il <= ilmin.  The budget is a countdown:
+	// `left` candidates of the B segment (chain / 4), then B's snapshot and `rest` candidates of the A segment.
+	const uint8_t *lb = reinterpret_cast<const uint8_t *>(s_link);
 	for (uint32_t i = threadIdx.x; i < total; i += kMatchThreads) {
 		const uint32_t p = t0 + (uint32_t)__ldcg(&order[i]);
-		uint32_t resA = 0, resB = 0;
 		const uint32_t la = n - p;
-		const uint32_t d = (uint32_t)s_link[p - w0];
-		if (d != 0) {
-			const uint32_t maxlen = la < (uint32_t)kMaxMatch ? la : (uint32_t)kMaxMatch;
-			const uint32_t nice = la < (uint32_t)lp.nice ? la : (uint32_t)lp.nice;
-			const uint32_t is = p - w0;
-			const uint8_t *sp = s_data + is;
-			uint32_t m = kMinMatch - 1, bd = 0, dist = d, cnt = 0;
-			bool haveB = false;
-			uint32_t stop = budgetB ? budgetB : chain;
-			const uint32_t s0 = sp[0], s1 = sp[1];
-			uint32_t scan_end1 = s1, scan_end = sp[2];
-			// bytes 2..9 of the scan string stay in registers: most extensions end inside them
-			uint32_t sw0, sw1;
-			{
-				const uint32_t as = is + 2;
-				const uint32_t *ws = reinterpret_cast<const uint32_t *>(s_data + (as & ~3u));
-				const uint32_t w1 = ws[1], sh = (as & 3u) * 8u;
-				sw0 = __funnelshift_r(ws[0], w1, sh);
-				sw1 = __funnelshift_r(w1, ws[2], sh);
-			}
-			for (;;) {
-				const uint32_t ic = is - dist;
-				const uint8_t *c = s_data + ic;
-				++cnt;
-				if (c[m] == scan_end && c[m - 1] == scan_end1 && c[0] == s0 && c[1] == s1) {
-					uint32_t l = 2;
-					if (maxlen >= 10) {
-						const uint32_t ac = ic + 2;
-						const uint32_t *wc = reinterpret_cast<const uint32_t *>(s_data + (ac & ~3u));
-						const uint32_t w1 = wc[1], sh = (ac & 3u) * 8u;
-						uint32_t x = __funnelshift_r(wc[0], w1, sh) ^ sw0;
-						if (x) {
-							l = 2 + ((uint32_t)(__ffs((int)x) - 1) >> 3);
-							goto lcp_done;
-						}
-						x = __funnelshift_r(w1, wc[2], sh) ^ sw1;
-						if (x) {
-							l = 6 + ((uint32_t)(__ffs((int)x) - 1) >> 3);
-							goto lcp_done;
-						}
-						l = 10;
-					}
-					while (l + 4 <= maxlen) {
-						const uint32_t ac = ic + l, as = is + l;
-						const uint32_t *wc = reinterpret_cast<const uint32_t *>(s_data + (ac & ~3u));
-						const uint32_t *ws = reinterpret_cast<const uint32_t *>(s_data + (as & ~3u));
-						const uint32_t x = __funnelshift_r(wc[0], wc[1], (ac & 3u) * 8u) ^ __funnelshift_r(ws[0], ws[1], (as & 3u) * 8u);
-						if (x) {
-							l += (uint32_t)(__ffs((int)x) - 1) >> 3;
-							goto lcp_done;
-						}
-						l += 4;
-					}
-					while (l < maxlen && c[l] == sp[l]) ++l;
-				lcp_done:
-					if (l > m) {
-						m = l;
-						bd = dist;
-						if (m >= nice) break;
-						scan_end1 = sp[m - 1];
-						scan_end = sp[m];
-					}
-				}
-				if (cnt == stop) { // one test per candidate: first the quarter budget (B's snapshot), then the full one
-					if (stop == chain) break;
-					resB = m >= (uint32_t)kMinMatch ? pack_match(m, bd) : 0u;
-					haveB = true;
-					stop = chain;
-				}
-				const uint32_t l2 = s_link[is - dist];
-				if (l2 == 0) break;
-				dist += l2;
-				if (dist >= (uint32_t)kMaxDist) break; // chain entries need distance < 32506 (T7)
-			}
-			resA = m >= (uint32_t)kMinMatch ? pack_match(m, bd) : 0u;
-			if (!haveB) resB = resA;
+		const uint32_t maxlen = la < (uint32_t)kMaxMatch ? la : (uint32_t)kMaxMatch;
+		const uint32_t nice = la < (uint32_t)lp.nice ? la : (uint32_t)lp.nice;
+		const uint32_t is = p - w0;
+		const uint8_t *sp = s_data + is;
+		// every position in the order has a first candidate: the class pass gave the others class 0
+		const int ic0 = (int)is - (int)s_link[is];
+		int icm = ic0 + (kMinMatch - 1), il = 2 * ic0;
+		const int ilmin = 2 * ((int)is - kMaxDist); // chain entries need distance < 32506 (T7)
+		uint32_t m = kMinMatch - 1, bd = 0, resB = 0;
+		bool haveB = false;
+		uint32_t left = budgetB ? budgetB : chain, rest = chain - left;
+		const uint32_t s0 = sp[0], s1 = sp[1];
+		uint32_t scan_end1 = s1, scan_end = sp[2];
+		// bytes 2..9 of the scan string stay in registers: most extensions end inside them
+		uint32_t sw0, sw1;
+		{
+			const uint32_t as = is + 2;
+			const uint32_t *ws = reinterpret_cast<const uint32_t *>(s_data + (as & ~3u));
+			const uint32_t w1 = ws[1], sh = (as & 3u) * 8u;
+			sw0 = __funnelshift_r(ws[0], w1, sh);
+			sw1 = __funnelshift_r(w1, ws[2], sh);
 		}
-		out[p] = make_uint2(resA, resB);
+		for (;;) { // the B segment, then the A segment
+			for (;;) { // one candidate
+				const uint32_t l2 = *reinterpret_cast<const uint16_t *>(lb + il);
+				if (s_data[icm] == scan_end && s_data[icm - 1] == scan_end1) {
+					const uint32_t ic = (uint32_t)(il >> 1);
+					const uint8_t *c = s_data + ic;
+					if (c[0] == s0 && c[1] == s1) {
+						uint32_t l = 2;
+						if (maxlen >= 10) {
+							const uint32_t ac = ic + 2;
+							const uint32_t *wc = reinterpret_cast<const uint32_t *>(s_data + (ac & ~3u));
+							const uint32_t w1 = wc[1], sh = (ac & 3u) * 8u;
+							uint32_t x = __funnelshift_r(wc[0], w1, sh) ^ sw0;
+							if (x) {
+								l = 2 + ((uint32_t)(__ffs((int)x) - 1) >> 3);
+								goto lcp_done;
+							}
+							x = __funnelshift_r(w1, wc[2], sh) ^ sw1;
+							if (x) {
+								l = 6 + ((uint32_t)(__ffs((int)x) - 1) >> 3);
+								goto lcp_done;
+							}
+							l = 10;
+						}
+						while (l + 4 <= maxlen) {
+							const uint32_t ac = ic + l, as = is + l;
+							const uint32_t *wc = reinterpret_cast<const uint32_t *>(s_data + (ac & ~3u));
+							const uint32_t *ws = reinterpret_cast<const uint32_t *>(s_data + (as & ~3u));
+							const uint32_t x = __funnelshift_r(wc[0], wc[1], (ac & 3u) * 8u) ^ __funnelshift_r(ws[0], ws[1], (as & 3u) * 8u);
+							if (x) {
+								l += (uint32_t)(__ffs((int)x) - 1) >> 3;
+								goto lcp_done;
+							}
+							l += 4;
+						}
+						while (l < maxlen && c[l] == sp[l]) ++l;
+					lcp_done:
+						if (l > m) {
+							m = l;
+							bd = is - ic;
+							if (m >= nice) goto walk_done;
+							scan_end1 = sp[m - 1];
+							scan_end = sp[m];
+							icm = (int)(ic + m);
+						}
+					}
+				}
+				icm -= (int)l2;
+				il -= 2 * (int)l2;
+				if ((il <= ilmin) | (--left == 0)) break;
+			}
+			if (il <= ilmin || rest == 0) break;
+			resB = m >= (uint32_t)kMinMatch ? pack_match(m, bd) : 0u; // B: the first chain / 4 candidates
+			haveB = true;
+			left = rest;
+			rest = 0;
+		}
+	walk_done:
+		const uint32_t resA = m >= (uint32_t)kMinMatch ? pack_match(m, bd) : 0u;
+		out[p] = make_uint2(resA, haveB ? resB : resA);
 	}
 }
 
@@ -1839,6 +1853,14 @@ int deflate_plan_run(b200z_plan *p, const uint8_t *d_in, uint8_t *d_out, int64_t
 	}
 	p->mark(s, "end");
 	B200Z_CUDA(cudaGetLastError());
+	return B200Z_OK;
+}
+
+int deflate_plan_match_table(b200z_plan *p, int32_t i, uint16_t *link, uint32_t *ab, cudaStream_t s) {
+	const int64_t off = p->in_off[i], n = p->in_len[i], H = p->hist.empty() ? 0 : p->hist[i];
+	if (link) B200Z_CUDA(cudaMemcpyAsync(link, p->ws.at<uint16_t>(p->o_link) + off, 2 * n, cudaMemcpyDeviceToHost, s));
+	B200Z_CUDA(cudaMemcpyAsync(ab, p->ws.at<uint2>(p->o_mt) + off + H, 8 * (n - H), cudaMemcpyDeviceToHost, s));
+	B200Z_CUDA(cudaStreamSynchronize(s));
 	return B200Z_OK;
 }
 

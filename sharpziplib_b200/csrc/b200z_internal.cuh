@@ -164,6 +164,7 @@ namespace b200z {
 int deflate_plan_build(b200z_plan *p);
 int deflate_plan_run(b200z_plan *p, const uint8_t *d_in, uint8_t *d_out, int64_t *d_out_len, int32_t *d_status,
                      uint32_t *d_check, int64_t *d_out_bits, cudaStream_t s, int stages);
+int deflate_plan_match_table(b200z_plan *p, int32_t i, uint16_t *link, uint32_t *ab, cudaStream_t s);
 int inflate_plan_build(b200z_plan *p);
 int inflate_plan_stats(b200z_plan *p, uint32_t *v, int32_t cap, cudaStream_t s);
 int inflate_plan_run(b200z_plan *p, const uint8_t *d_in, uint8_t *d_out, int64_t *d_out_len, int32_t *d_status,

@@ -5,7 +5,8 @@
 //   * candidates the reference walks (only at the positions DeflateSlow visits, with the carried threshold and budget)
 //   * how often a candidate passes the first quick-reject byte / the whole quick reject / improves the match
 // build: g++ -O2 -std=c++17 -I sharpziplib_b200/csrc -o /tmp/match_stats tools/match_stats.cpp
-// run:   /tmp/match_stats <file of concatenated buffers> <buffer size> <level>
+// run:   /tmp/match_stats <file of concatenated buffers> <buffer size> <level> [reuse]
+//        (with "reuse": only the count of extension work that position p+1's result could replace)
 #include "b200z_core.cuh"
 #include <cstdio>
 #include <cstdlib>
@@ -77,6 +78,72 @@ static uint32_t walk(const uint8_t *data, const uint16_t *link, uint32_t p, uint
 	return m > m0 ? pack_match(m, bd) : 0;
 }
 
+// k_match's extension after a passed quick reject: the two register compares of bytes 2..9, then the loop of 4-byte compares
+// and the byte tail.  Returns the lcp; `words` gets the iterations of the 4-byte loop plus the tail's byte steps.
+static uint32_t kernel_extension(const uint8_t *s, const uint8_t *c, uint32_t maxlen, uint64_t &words) {
+	uint32_t l = 2;
+	if (maxlen >= 10) {
+		while (l < 10 && c[l] == s[l]) ++l;
+		if (l < 10) return l;
+	}
+	while (l + 4 <= maxlen) {
+		++words;
+		uint32_t k = 0;
+		while (k < 4 && c[l + k] == s[l + k]) ++k;
+		l += k;
+		if (k < 4) return l;
+	}
+	while (l < maxlen && c[l] == s[l]) {
+		++words;
+		++l;
+	}
+	return l;
+}
+
+// How much of k_match's extension loop the lcp of position p+1 could replace: for a candidate at p+1's best distance d
+// that passes the quick reject, lcp(p, d) = min(lcp(p + 1, d) + 1, maxlen(p)) without extending.  Counted as if every
+// position's predecessor p+1 ran on the same thread just before it (an upper bound: the class order splits some pairs).
+static void reuse_stats(const uint8_t *data, const uint16_t *link, uint32_t n, const LevelParams &lp, uint64_t &words,
+                        uint64_t &reusable, uint64_t &hits) {
+	uint32_t prev_d = 0, prev_l = 0; // p+1's best distance and its full capped lcp (0: none)
+	for (uint32_t p = n; p-- > 0;) {
+		const uint32_t la = n - p;
+		uint32_t d = la >= (uint32_t)kMinMatch ? link[p] : 0u;
+		uint32_t best_d = 0, m = kMinMatch - 1;
+		if (d != 0 && d <= (uint32_t)kMaxDist) {
+			const uint32_t maxlen = la < (uint32_t)kMaxMatch ? la : (uint32_t)kMaxMatch;
+			const uint32_t nice = la < (uint32_t)lp.nice ? la : (uint32_t)lp.nice;
+			const uint8_t *s = data + p;
+			uint32_t dist = d, cnt = 0;
+			for (;;) {
+				const uint8_t *c = s - dist;
+				++cnt;
+				if (c[m] == s[m] && c[m - 1] == s[m - 1] && c[0] == s[0] && c[1] == s[1]) {
+					uint64_t w = 0;
+					const uint32_t l = kernel_extension(s, c, maxlen, w);
+					words += w;
+					if (dist == prev_d && prev_l) {
+						reusable += w;
+						hits++;
+					}
+					if (l > m) {
+						m = l;
+						best_d = dist;
+						if (m >= nice) break;
+					}
+				}
+				if (cnt == (uint32_t)lp.chain) break;
+				const uint32_t l2 = link[p - dist];
+				if (l2 == 0) break;
+				dist += l2;
+				if (dist >= (uint32_t)kMaxDist) break;
+			}
+		}
+		prev_d = best_d;
+		prev_l = best_d ? m : 0;
+	}
+}
+
 int main(int argc, char **argv) {
 	if (argc < 4) return 1;
 	FILE *f = fopen(argv[1], "rb");
@@ -84,6 +151,18 @@ int main(int argc, char **argv) {
 	const int level = atoi(argv[3]);
 	const LevelParams lp = level_params(level);
 	std::vector<uint8_t> buf(bs + 16);
+	if (argc > 4) { // "reuse": only this count
+		uint64_t words = 0, reusable = 0, hits = 0;
+		while (fread(buf.data(), 1, bs, f) == bs) {
+			std::vector<uint16_t> link;
+			links(buf.data(), bs, link);
+			reuse_stats(buf.data(), link.data(), bs, lp, words, reusable, hits);
+		}
+		printf("extension reuse from p+1: %llu of %llu word steps of the extension loop (%.1f%%) fall on p+1's best distance "
+		       "(%llu candidates)\n", (unsigned long long)reusable, (unsigned long long)words, 100.0 * reusable / (words ? words : 1),
+		       (unsigned long long)hits);
+		return 0;
+	}
 	Cnt all, ref;
 	uint64_t visited = 0, used_a = 0, used_b = 0, useful = 0, nsym = 0;
 	int nb = 0;
